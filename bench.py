@@ -374,6 +374,28 @@ def reduce_timing(values, dist, device):
     return [float(x) for x in t]
 
 
+DUMP_BYTES = 60_000_000  # what --dump-outputs writes in all (npy headers aside)
+
+
+def dump_outputs(out_dir, torch, dv, n):
+    """The outputs of the last timed step, for comparing two builds: for every
+    frame, the reconstructed colour and reflectance at a fixed, seeded sample of
+    points and the colour and reflectance coefficients at the same positions of
+    the coefficient planes (coding order), as float32 (attributes) and float64
+    (coefficients).  The sample is sized to keep the files under DUMP_BYTES."""
+    k = min(n, DUMP_BYTES // (len(dv) * (4 * 4 + 4 * 8)))
+    idx = np.sort(np.random.default_rng(0).choice(n, size=k, replace=False))
+    ti = torch.from_numpy(idx).to(dv[0]["rgb"].device)
+    planes = {"rgb": (lambda d: d["rgb"][ti], np.float32),
+              "reflectance": (lambda d: d["refl"][ti], np.float32),
+              "coef_rgb": (lambda d: d["crgb"][:, ti], np.float64),
+              "coef_reflectance": (lambda d: d["crefl"][:, ti], np.float64)}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, (take, dtype) in planes.items():
+        a = torch.stack([take(d) for d in dv]).cpu().numpy().astype(dtype)
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 # ---------------------------------------------------------------------------
 # our arm
 
@@ -476,6 +498,8 @@ def run_ours(args):
     launches = pb.kernel_launch_count() - launches0
     barrier()
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, torch, dv, n)
 
     # latency of one frame alone
     single_ms = min(timed_device_step(dv[:1]) for _ in range(3))
@@ -846,7 +870,12 @@ def main():
     ap.add_argument("--frames", type=int, default=FRAMES_PER_STEP,
                     help="independent frames in flight per GPU per step (intra coding: frames "
                          "are independent work units)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write a seeded sample of the last timed step's reconstructions and "
+                         "coefficients, every frame, to DIR/*.npy (inputs are the same on every run)")
     args = ap.parse_args()
+    if args.dump_outputs and (args.workload != "raht1m" or args.impl != "ours"):
+        ap.error("--dump-outputs applies to the raht1m workload of --impl ours")
     if args.workload != "raht1m":
         import bench_workloads
 

@@ -1,15 +1,19 @@
 """Generate the committed golden vectors from the UNMODIFIED reference.
 
-Run in the build container (needs /root/reference compiled into
-oracle/_ref/libtmc13_ref.so by `make -C oracle ref`):
+Needs the compiled reference in oracle/_ref (`make -C oracle ref liftref
+recolourref REF=<reference source tree>`):
 
     python tests/golden/make_golden.py
 
 Writes tests/golden/raht_golden.npz (inputs + reference outputs for a set of
-small clouds x parameter variants) and tests/golden/arith_golden.npz
-(known-answer vectors of the scalar helpers).  The GPU box has no
-/root/reference: tests there read these files only."""
+small clouds x parameter variants), tests/golden/arith_golden.npz
+(known-answer vectors of the scalar helpers), the LoD, spherical and symbol
+vectors, and tests/golden/reference_tape.npz (what the reference returned to
+every ref_* call of the suite's comparisons, see pcc_testlib.taped).  The
+comparisons read these files only: they need neither the reference sources
+nor oracle/_ref."""
 import os
+import subprocess
 import sys
 
 import numpy as np
@@ -118,7 +122,23 @@ def main():
     np.savez_compressed(os.path.join(HERE, "lod_golden.npz"), **lod)
     spherical_golden()
     symbols_golden()
+    record_reference_tape()
     print("golden vectors written")
+
+
+# the tests whose ref_* calls the tape serves (the fuzz slices record from
+# their subprocesses)
+TAPED_TESTS = ["tests/test_oracle_vs_reference.py", "tests/test_recolour.py", "tests/test_fuzz_cpu.py"]
+
+
+def record_reference_tape():
+    """run the comparisons against the compiled reference and record its outputs"""
+    root = os.path.dirname(os.path.dirname(HERE))
+    if os.path.exists(TAPE_PATH):
+        os.remove(TAPE_PATH)
+    env = dict(os.environ, PCCB200_RECORD_REFERENCE="1")
+    subprocess.check_call([sys.executable, "-m", "pytest", "-q", "-p", "no:cacheprovider", *TAPED_TESTS],
+                          cwd=root, env=env)
 
 
 SYMBOL_GOLDEN_CASES = [("shell3", 3, 16), ("shell1", 1, 22), ("lidar3", 3, 28), ("lidar1", 1, 10)]

@@ -1,12 +1,19 @@
 """Shared test helpers: ctypes views of the C-ABI PODs, loaders for the
 oracle (oracle/liboracle.so) and the compiled reference
-(oracle/_ref/libtmc13_ref.so), and the synthetic point-cloud generators of
-SURVEY.md 8(d).  TEST INFRASTRUCTURE ONLY."""
+(oracle/_ref/libtmc13_ref.so), the recorded outputs of that reference
+(tests/golden/reference_tape.npz), and the synthetic point-cloud generators
+of SURVEY.md 8(d).  TEST INFRASTRUCTURE ONLY."""
+import atexit
 import ctypes as C
+import functools
+import hashlib
+import inspect
+import json
 import os
 import subprocess
 
 import numpy as np
+from numpy.lib.recfunctions import structured_to_unstructured
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 ORACLE_DIR = os.path.join(ROOT, "oracle")
@@ -179,6 +186,162 @@ def load_ref():
     return _ref
 
 
+# --------------------------------------------------------------------------
+# recorded outputs of the compiled reference
+#
+# The reference is only available where its sources are, so every ref_*
+# function below replays what it returned when it was recorded
+# (tests/golden/make_golden.py runs the suite with PCCB200_RECORD_REFERENCE=1
+# and the compiled reference present).  Entries are keyed by the function and
+# a digest of its arguments, so a test whose inputs drift fails instead of
+# comparing against another case.  Large arrays are kept as digests
+# (`Recorded`, compared with `same`), small ones and scalars by value.  Inputs
+# that were never recorded go to the compiled reference when it is present.
+
+TAPE_PATH = os.path.join(ROOT, "tests", "golden", "reference_tape.npz")
+RECORDING = os.environ.get("PCCB200_RECORD_REFERENCE") == "1"
+_BY_VALUE_BYTES = 256
+_tape = None
+
+
+class Recorded:
+    """an array the reference returned, known by its digest (see `digest`)"""
+
+    def __init__(self, sha256, shape):
+        self.sha256, self.shape = sha256, tuple(shape)
+
+    def __repr__(self):
+        return f"Recorded(shape={self.shape}, sha256={self.sha256[:12]}...)"
+
+
+def digest(x):
+    """sha256 (first 128 bits) of an integer array's shape and values (the
+    dtype does not count: equal digests <=> np.array_equal); bytes count as a
+    uint8 array"""
+    if isinstance(x, Recorded):
+        return x.sha256
+    if isinstance(x, (bytes, bytearray)):
+        x = np.frombuffer(x, dtype=np.uint8)
+    x = np.asarray(x)
+    if x.dtype.names:  # predictors: one column per field element
+        x = structured_to_unstructured(x)
+    if x.dtype.kind not in "iub":
+        raise TypeError(f"digest of a {x.dtype} array")
+    v = x.astype(np.uint64).view(np.int64) if x.dtype == np.uint64 else x.astype(np.int64)
+    h = hashlib.sha256(repr(x.shape).encode())
+    h.update(np.ascontiguousarray(v).tobytes())
+    return h.hexdigest()[:32]
+
+
+def same(*xs):
+    """all arguments (arrays, bytes, Recorded) hold the same values"""
+    return len({digest(x) for x in xs}) == 1
+
+
+def _token(a):
+    if a is None or isinstance(a, (bool, str)):
+        return repr(a)
+    if isinstance(a, (int, np.integer)):
+        return repr(int(a))
+    if isinstance(a, (float, np.floating)):
+        return repr(float(a))
+    if isinstance(a, C.Structure):
+        return "pod:" + bytes(a).hex()
+    if isinstance(a, (tuple, list)):
+        return "(" + ",".join(_token(x) for x in a) + ")"
+    return "array:" + digest(a)
+
+
+def _encode(out, name, arrays, by_value):
+    if isinstance(out, tuple):
+        return {"tuple": [_encode(x, f"{name}/{i}", arrays, by_value) for i, x in enumerate(out)]}
+    if isinstance(out, (bytes, bytearray)):
+        return {"sha256": digest(out), "shape": [len(out)]}
+    if isinstance(out, np.ndarray):
+        if out.nbytes <= _BY_VALUE_BYTES and not out.dtype.names:
+            return {"list": out.tolist(), "dtype": out.dtype.str}
+        if by_value:  # stored in the narrowest integer type that holds it
+            arrays[name] = out.astype(np.result_type(np.min_scalar_type(out.min()), np.min_scalar_type(out.max())))
+            return {"array": name, "dtype": out.dtype.str}
+        return {"sha256": digest(out), "shape": list(out.shape)}
+    if isinstance(out, list):
+        return {"value": [int(x) for x in out]}
+    return {"value": out.item() if isinstance(out, np.generic) else out}
+
+
+def _decode(e, arrays):
+    if "tuple" in e:
+        return tuple(_decode(x, arrays) for x in e["tuple"])
+    if "array" in e:
+        return arrays[e["array"]].astype(e["dtype"])
+    if "list" in e:
+        return np.array(e["list"], dtype=e["dtype"])
+    if "sha256" in e:
+        return Recorded(e["sha256"], e["shape"])
+    return e["value"]
+
+
+def _read_tape():
+    if not os.path.exists(TAPE_PATH):
+        return {}, {}
+    with np.load(TAPE_PATH) as z:
+        return json.loads(z["index"].tobytes()), {k: z[k] for k in z.files if k != "index"}
+
+
+def _save_tape():
+    """merge this process's recordings into the tape (the fuzz tools record
+    from subprocesses of the test run)"""
+    index, arrays = _read_tape()
+    index.update(_tape[0])
+    arrays.update(_tape[1])
+    text = json.dumps(index, sort_keys=True, separators=(",", ":")).encode()
+    np.savez_compressed(TAPE_PATH, index=np.frombuffer(text, dtype=np.uint8), **arrays)
+
+
+def _load_tape():
+    global _tape
+    if _tape is None:
+        if RECORDING:
+            _tape = ({}, {})
+            atexit.register(_save_tape)
+        else:
+            _tape = _read_tape()
+    return _tape
+
+
+def taped(by_value=False):
+    """replay (or, when recording, record) the outputs of a ref_* function;
+    by_value keeps whole arrays, for tests that measure how far the oracle
+    is from the reference rather than asserting equality"""
+
+    def wrap(fn):
+        sig = inspect.signature(fn)
+
+        @functools.wraps(fn)
+        def call(*args, **kw):
+            bound = sig.bind(*args, **kw)
+            bound.apply_defaults()
+            key = hashlib.sha256((fn.__name__ + _token(tuple(bound.arguments.values()))).encode()).hexdigest()[:32]
+            index, arrays = _load_tape()
+            if not RECORDING and key in index:
+                return _decode(index[key], arrays)
+            if any(isinstance(a, Recorded) for a in bound.arguments.values()):
+                raise LookupError(f"{fn.__name__}: no recorded output for these inputs")
+            try:
+                out = fn(*bound.args, **bound.kwargs)
+            except OSError as e:
+                raise LookupError(
+                    f"{fn.__name__}: no recorded output for these inputs and no compiled reference in "
+                    "oracle/_ref; re-record with tests/golden/make_golden.py") from e
+            if RECORDING:
+                index[key] = _encode(out, key, arrays, by_value)
+            return out
+
+        return call
+
+    return wrap
+
+
 def _run_raht(fn, forward, params, qpset, morton, attrs, coeffs, qpoffs):
     n, a = attrs.shape
     attrs = np.ascontiguousarray(attrs, dtype=np.int32).copy()
@@ -204,6 +367,7 @@ def oracle_raht(forward, params, qpset, morton, attrs, coeffs=None, qpoffs=None)
     return a, c
 
 
+@taped()
 def ref_raht(forward, params, qpset, morton, attrs, coeffs=None, qpoffs=None,
              want_time=False):
     a, c, t = _run_raht(load_ref().tmc13ref_raht, forward, params, qpset,
@@ -221,6 +385,7 @@ def oracle_morton_sort(xyz):
     return keys, order
 
 
+@taped()
 def ref_morton_sort(xyz):
     xyz = np.ascontiguousarray(xyz, dtype=np.int32)
     n = xyz.shape[0]
@@ -229,6 +394,15 @@ def ref_morton_sort(xyz):
     load_ref().tmc13ref_morton_sort(_ptr(xyz, C.c_int32), C.c_int(n),
                                     _ptr(keys, C.c_int64), _ptr(order, C.c_int32))
     return keys, order
+
+
+@taped()
+def ref_elementwise(name, dtype, *columns):
+    """the reference's scalar helper tmc13ref_<name> applied to every row of
+    the argument columns -> array of `dtype`"""
+    lib = load_ref() if name != "iatan2" else _load_liftref()
+    f = getattr(lib, "tmc13ref_" + name)
+    return np.array([f(*map(int, row)) for row in zip(*columns)], dtype=dtype)
 
 
 import sys as _sys
@@ -339,12 +513,14 @@ def oracle_lift(forward, preds, qw, npl, attrs):
     return a
 
 
+@taped()
 def ref_quant_weights(preds):
     qw = np.zeros(preds.shape[0], dtype=np.uint64)
     load_ref().tmc13ref_quant_weights(_pp(preds), C.c_int(preds.shape[0]), _ptr(qw, C.c_uint64))
     return qw
 
 
+@taped()
 def ref_lift(forward, preds, qw, npl, attrs):
     a = np.ascontiguousarray(attrs, dtype=np.int64).copy()
     if a.ndim == 1:
@@ -409,6 +585,7 @@ def _run_lod(fn, params, xyz):
     return preds, indexes, npl[:cnt.value].copy(), r
 
 
+@taped()
 def ref_lod_build(params, xyz):
     load_ref().tmc13ref_lod_build.restype = C.c_double
     p, i, n, t = _run_lod(load_ref().tmc13ref_lod_build, params, xyz)
@@ -441,6 +618,7 @@ def liftref_available():
     return os.path.exists(os.path.join(ORACLE_DIR, "_ref", "libtmc13_lift.so"))
 
 
+@taped()
 def ref_lift_encode(lod_params, qpset, lcp_enabled, xyz, attrs, bitdepth=8):
     """The reference's own lifting encoder (LoD build, weights, forward lifting,
     quantisation (+LCP), reconstruction): -> (values [N,A] predictor order,
@@ -558,6 +736,7 @@ def _run_rpl(fn, origin, theta, xyz, weight=None, min_pos=None, emu=False):
     return out, bbox
 
 
+@taped()
 def ref_xyz_to_rpl(origin, theta, xyz):
     return _run_rpl(_load_liftref().tmc13ref_xyz_to_rpl, origin, theta, xyz)
 
@@ -576,6 +755,7 @@ def _run_offset_scale(fn, min_pos, weight, pos):
     return pos
 
 
+@taped()
 def ref_offset_and_scale(min_pos, weight, pos):
     return _run_offset_scale(_load_liftref().tmc13ref_offset_and_scale, min_pos, weight, pos)
 
@@ -584,6 +764,7 @@ def oracle_offset_and_scale(min_pos, weight, pos):
     return _run_offset_scale(load_oracle().oracle_offset_and_scale, min_pos, weight, pos)
 
 
+@taped()
 def ref_normalised_axes_weights(box_max, forced_max_log2=0):
     out = (C.c_int32 * 3)()
     _load_liftref().tmc13ref_normalised_axes_weights(_i3(box_max), C.c_int(forced_max_log2), out)
@@ -620,6 +801,7 @@ def emu_coeff_symbols(coeffs):
     return _run_symbols(load_emu().emu_coeff_symbols, coeffs)
 
 
+@taped()
 def ref_raht_encode_payload(params, qpset, xyz, attrs, bitdepth=8):
     """the reference's own RAHT attribute encoder (sort, transform, coefficient
     walk, arithmetic coding) -> (payload bytes, reconstruction [N, A])"""
@@ -638,6 +820,7 @@ def ref_raht_encode_payload(params, qpset, xyz, attrs, bitdepth=8):
     return bytes(buf[:ln]), recon
 
 
+@taped()
 def ref_symbols_payload(mode, runs, values, ctx, tail, n):
     """a symbol stream through the reference's PCCResidualsEncoder -> payload bytes
     (mode 0: its encode() members; mode 1: encodeSymbol with the given selectors)"""
@@ -656,6 +839,7 @@ def ref_symbols_payload(mode, runs, values, ctx, tail, n):
     return bytes(buf[:ln])
 
 
+@taped()
 def ref_decode_symbol_stream(payload, n, a):
     """the symbol stream as the reference's RAHT decoder reads it"""
     lib = _load_liftref()
@@ -680,6 +864,7 @@ def _run_dist2(fn, xyz, period, rng_, pct):
               C.c_float(pct))
 
 
+@taped()
 def ref_estimate_dist2(xyz, period=100, search_range=128, pct=0.85):
     return _run_dist2(_load_liftref().tmc13ref_estimate_dist2, xyz, period, search_range, pct)
 
@@ -695,6 +880,7 @@ def emu_estimate_dist2(xyz, period=100, search_range=128, pct=0.85):
 # --------------------------------------------------------------------------
 # the other two quantisation-weight derivations (row L5)
 
+@taped()
 def ref_quant_weights_fixed(preds, neigh_weight):
     qw = np.zeros(preds.shape[0], dtype=np.uint64)
     load_ref().tmc13ref_quant_weights_fixed(_pp(preds), C.c_int(preds.shape[0]), _i3(neigh_weight),
@@ -720,6 +906,7 @@ def emu_quant_weights_fixed(preds, npl, neigh_weight):
     return qw
 
 
+@taped()
 def ref_quant_weights_scalable(preds, npl, num_points, min_log2):
     npl = np.ascontiguousarray(npl, dtype=np.uint32)
     qw = np.zeros(preds.shape[0], dtype=np.uint64)
@@ -805,6 +992,7 @@ def recolourref_available():
     return os.path.exists(os.path.join(ORACLE_DIR, "_ref", "libtmc13_recolour.so"))
 
 
+@taped(by_value=True)
 def ref_recolour(params, sxyz, sattr, scale, off, txyz, bitdepth=8):
     global _recolourref
     if _recolourref is None:

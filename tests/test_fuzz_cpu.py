@@ -1,23 +1,18 @@
 """Seeded slices of the CPU fuzzers (tools/fuzz_cpu.py, tools/fuzz_lod_cpu.py,
 tools/fuzz_misc_cpu.py):
 compiled reference == oracle == kernel bodies (host build) over random points
-of the parameter space.  The full sweeps are developer tools; these keep a few
-dozen configurations in the regular suite."""
+of the parameter space, the reference's outputs replayed from
+tests/golden/reference_tape.npz.  The full sweeps are developer tools; these
+keep a few dozen configurations in the regular suite."""
 import os
 import subprocess
 import sys
 
 import pytest
 
-from pcc_testlib import ORACLE_DIR
-
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-needs_ref = pytest.mark.skipif(
-    not os.path.exists(os.path.join(ORACLE_DIR, "_ref", "libtmc13_ref.so")),
-    reason="oracle/_ref/libtmc13_ref.so not built (make -C oracle ref)")
 
 
-@needs_ref
 @pytest.mark.parametrize("tool,cases,seed", [("fuzz_cpu.py", 40, 101), ("fuzz_lod_cpu.py", 30, 102),
                                              ("fuzz_misc_cpu.py", 30, 103)])
 def test_fuzz_slice(tool, cases, seed):

@@ -1,7 +1,7 @@
 """CPU tests: the oracle (oracle/raht_oracle.c) against (a) the committed
-golden vectors produced by the unmodified reference and (b), when the
-compiled reference is present (oracle/_ref), the reference run live on a
-wider set of clouds and flag combinations."""
+golden vectors produced by the unmodified reference and (b) the outputs of
+the compiled reference on a wider set of clouds and flag combinations, as
+recorded in tests/golden/reference_tape.npz (pcc_testlib: `taped`)."""
 import os
 
 import numpy as np
@@ -56,23 +56,19 @@ def test_raht_golden(raht_gold, cname):
             assert np.array_equal(rec2, rec), (vname, qp)
 
 
-needs_ref = pytest.mark.skipif(not ref_available(), reason="compiled reference (oracle/_ref) not present")
-
-
 def _cmp(xyz, attrs, p, qs, qpo=None):
     mort, a_s, order = sort_cloud(xyz, attrs)
     q = qpo[order] if qpo is not None else None
     rr, rc = ref_raht(1, p, qs, mort, a_s, qpoffs=q)
     orr, oc = oracle_raht(1, p, qs, mort, a_s, qpoffs=q)
-    assert np.array_equal(rc, oc)
-    assert np.array_equal(rr, orr)
+    assert same(rc, oc)
+    assert same(rr, orr)
     r2, _ = ref_raht(0, p, qs, mort, a_s * 0, coeffs=rc, qpoffs=q)
-    o2, _ = oracle_raht(0, p, qs, mort, a_s * 0, coeffs=rc, qpoffs=q)
-    assert np.array_equal(r2, o2)
-    assert np.array_equal(r2, rr)  # decoder reproduces the encoder's reconstruction
+    o2, _ = oracle_raht(0, p, qs, mort, a_s * 0, coeffs=oc, qpoffs=q)
+    assert same(r2, o2)
+    assert same(r2, rr)  # decoder reproduces the encoder's reconstruction
 
 
-@needs_ref
 @pytest.mark.parametrize("kw", [dict(), dict(prediction=0), dict(subnode=0), dict(haar=1),
                                 dict(ext=0), dict(ext=0, subnode=0), dict(thr0=0, thr1=1)])
 @pytest.mark.parametrize("qp", [10, 34, 46])
@@ -81,7 +77,6 @@ def test_live_shell(kw, qp):
     _cmp(xyz, attrs, make_params(**kw), make_qpset(qp=qp))
 
 
-@needs_ref
 @pytest.mark.parametrize("a", [1, 3])
 def test_live_dups_and_lidar(a):
     xyz, attrs = cloud_shell(30000, bits=7, seed=4, a=a, dups=True)
@@ -93,7 +88,6 @@ def test_live_dups_and_lidar(a):
     _cmp(xyz, attrs, make_params(), make_qpset(qp=34))
 
 
-@needs_ref
 def test_live_qp_structures():
     rng = np.random.default_rng(7)
     xyz, attrs = cloud_shell(30000, bits=8, seed=5)
@@ -106,7 +100,6 @@ def test_live_qp_structures():
     _cmp(xyz, a16, make_params(), make_qpset(qp=40, bitdepth=16))
 
 
-@needs_ref
 def test_live_edge_cases():
     rng = np.random.default_rng(3)
     for n in (1, 2, 3, 9, 17):
@@ -122,19 +115,20 @@ def test_live_edge_cases():
         _cmp(xyz, attrs, make_params(thr0=0, thr1=1), make_qpset(qp=30))
 
 
-@needs_ref
 def test_live_scalar_helpers():
-    o, r = load_oracle(), load_ref()
+    o = load_oracle()
     rng = np.random.default_rng(5)
-    for x in list(range(0, 3000)) + [int(v) for v in rng.integers(0, 1 << 62, size=3000, dtype=np.uint64)]:
-        assert o.oracle_isqrt(x) == r.tmc13ref_isqrt(x)
-        assert o.oracle_irsqrt(x) == r.tmc13ref_irsqrt(x)
+    xs = np.concatenate([np.arange(0, 3000, dtype=np.uint64), rng.integers(0, 1 << 62, size=3000, dtype=np.uint64)])
+    assert same(ref_elementwise("isqrt", "uint64", xs),
+                np.array([o.oracle_isqrt(int(x)) for x in xs], dtype=np.uint64))
+    assert same(ref_elementwise("irsqrt", "uint64", xs),
+                np.array([o.oracle_irsqrt(int(x)) for x in xs], dtype=np.uint64))
     # kDivApproxDivisor[i] + 1 == 65536 // (i + 1) for every index the LUT serves
-    for b in range(1, 257):
-        assert o.oracle_div_approx(1 << 20, b, 0) == r.tmc13ref_div_approx(1 << 20, b, 0)
+    b = np.arange(1, 257)
+    assert same(ref_elementwise("div_approx", "int64", np.full(256, 1 << 20), b, np.zeros(256, dtype=np.int64)),
+                np.array([o.oracle_div_approx(1 << 20, int(v), 0) for v in b], dtype=np.int64))
 
 
-@needs_ref
 @pytest.mark.parametrize("a", [1, 3])
 def test_live_lifting(a):
     """lift_oracle.c against PCCComputeQuantizationWeights / PCCLiftPredict /
@@ -144,14 +138,14 @@ def test_live_lifting(a):
         preds, npl = synth_predictors(n, lods, seed=n)
         qw_r = ref_quant_weights(preds)
         qw_o = oracle_quant_weights(preds)
-        assert np.array_equal(qw_r, qw_o)
+        assert same(qw_r, qw_o)
         attrs = (rng.integers(0, 256, size=(n, a)).astype(np.int64)) << 8
         fr = ref_lift(1, preds, qw_r, npl, attrs)
         fo = oracle_lift(1, preds, qw_o, npl, attrs)
-        assert np.array_equal(fr, fo)
+        assert same(fr, fo)
         ir = ref_lift(0, preds, qw_r, npl, fr)
         io = oracle_lift(0, preds, qw_o, npl, fo)
-        assert np.array_equal(ir, io)
+        assert same(ir, io)
 
 
 LOD_CASES = [
@@ -170,12 +164,11 @@ def _cmp_lod(xyz, kw):
     lp = make_lod_params(**kw)
     rp, ri, rn = ref_lod_build(lp, xyz)
     op, oi, on = oracle_lod_build(lp, xyz)
-    assert np.array_equal(rn, on), kw
-    assert np.array_equal(ri, oi), kw
-    assert np.array_equal(rp, op), kw
+    assert same(rn, on), kw
+    assert same(ri, oi), kw
+    assert same(rp, op), kw
 
 
-@needs_ref
 @pytest.mark.parametrize("kw", LOD_CASES)
 def test_live_lod(kw):
     """lod_oracle.c against AttributeLods::generate of the compiled reference:
@@ -186,7 +179,6 @@ def test_live_lod(kw):
     _cmp_lod(xyz, dict(kw, levels=8))
 
 
-@needs_ref
 def test_live_lod_edge_cases():
     xyz, _ = cloud_random(20000, 21, seed=5, dup_frac=0.1)   # many atlases, stalled fill cursor
     _cmp_lod(xyz, dict(levels=14))
@@ -211,11 +203,6 @@ def test_lod_golden():
             assert np.array_equal(p, g[f"{cname}/{i}/preds"])
 
 
-needs_liftref = pytest.mark.skipif(not liftref_available(),
-                                   reason="oracle/_ref/libtmc13_lift.so not built (make -C oracle liftref)")
-
-
-@needs_liftref
 @pytest.mark.parametrize("a", [1, 3])
 def test_live_lifting_encoder(a):
     """The oracle chain (LoD build, weights, lifting, LCP, quantisation,
@@ -232,9 +219,9 @@ def test_live_lifting_encoder(a):
                     qs = make_qpset(qp=qp, chroma_offset=-2 if a == 3 else 0, fixed_point_qp_offset=24)
                     rv, rr, rl = ref_lift_encode(lp, qs, lcp, xyz, attrs)
                     ov, orr, ol = oracle_lift_encode(lp, qs, lcp, xyz, attrs)
-                    assert np.array_equal(rv, ov) and np.array_equal(rr, orr)
+                    assert same(rv, ov) and same(rr, orr)
                     if a == 3 and lcp:
-                        assert np.array_equal(rl, ol)
+                        assert same(rl, ol)
 
 
 # --------------------------------------------------------------------------
@@ -250,17 +237,16 @@ def test_spherical_golden():
         assert np.array_equal(sc, g[f"{name}/scaled"])
 
 
-@needs_liftref
 def test_live_spherical():
-    lib, orc = _load_liftref_for_test(), load_oracle()
+    orc = load_oracle()
     rng = np.random.default_rng(5)
     # the fixed-point arc tangent, all quadrants, axes, tiny and large arguments
     ys = np.concatenate([rng.integers(-(1 << 30), 1 << 30, 4000), rng.integers(-300, 300, 2000),
                          [0, 0, 1, -1, 5, -5, 0, (1 << 30), -(1 << 30)]])
     xs = np.concatenate([rng.integers(-(1 << 30), 1 << 30, 4000), rng.integers(-300, 300, 2000),
                          [0, 7, 0, 0, 5, 5, -9, (1 << 30), (1 << 30)]])
-    for y, x in zip(ys, xs):
-        assert orc.oracle_iatan2(int(y), int(x)) == lib.tmc13ref_iatan2(int(y), int(x)), (y, x)
+    assert same(ref_elementwise("iatan2", "int64", ys, xs),
+                np.array([orc.oracle_iatan2(int(y), int(x)) for y, x in zip(ys, xs)], dtype=np.int64))
     # whole conversion on LiDAR-shaped and uniformly random clouds
     xyz, _ = cloud_lidar(30000, seed=4)
     wide = rng.integers(-(1 << 21), 1 << 21, size=(20000, 3)).astype(np.int32)
@@ -272,15 +258,10 @@ def test_live_spherical():
                                (wide[:1], (1, 2, 3), lidar_lasers(5))):
         r, rb = ref_xyz_to_rpl(origin, theta, pts)
         o, ob = oracle_xyz_to_rpl(origin, theta, pts)
-        assert np.array_equal(r, o) and np.array_equal(rb, ob)
+        assert same(r, o) and same(rb, ob)
         w = ref_normalised_axes_weights(np.maximum(rb[3:], 1))
         for mp in (rb[:3], (0, 0, 0), (-50, 7, 1)):
-            assert np.array_equal(ref_offset_and_scale(mp, w, r), oracle_offset_and_scale(mp, w, o))
-
-
-def _load_liftref_for_test():
-    from pcc_testlib import _load_liftref
-    return _load_liftref()
+            assert same(ref_offset_and_scale(mp, w, r), oracle_offset_and_scale(mp, w, o))
 
 
 # --------------------------------------------------------------------------
@@ -308,7 +289,6 @@ def test_symbols_golden():
         assert (ctx is None) == (a == 1)
 
 
-@needs_liftref
 @pytest.mark.parametrize("a", [1, 3])
 def test_live_symbols(a):
     """the oracle's symbol stream, pushed through the reference's own
@@ -321,12 +301,12 @@ def test_live_symbols(a):
             params, qs = make_params(**kw), make_qpset(qp=qp)
             payload, recon = ref_raht_encode_payload(params, qs, xyz, attrs)
             rec, (runs, vals, ctx, tail) = _oracle_symbols_for(xyz, attrs, params, qs)
-            assert np.array_equal(rec, recon)
+            assert same(rec, recon)
             n = len(xyz)
-            assert ref_symbols_payload(0, runs, vals, ctx, tail, n) == payload
-            assert ref_symbols_payload(1, runs, vals, ctx, tail, n) == payload
+            assert same(ref_symbols_payload(0, runs, vals, ctx, tail, n), payload)
+            assert same(ref_symbols_payload(1, runs, vals, ctx, tail, n), payload)
             rr, rv, rt = ref_decode_symbol_stream(payload, n, a)
-            assert np.array_equal(rr, runs) and np.array_equal(rv, vals) and rt == tail
+            assert same(rr, runs) and same(rv, vals) and rt == tail
 
 
 # --------------------------------------------------------------------------
@@ -349,7 +329,6 @@ def _dist2_cases():
 DIST2_PARAMS = [(100, 128, 0.85), (1, 4, 0.5), (7, 1, 0.0), (10, 300, 0.99), (1000, 128, 0.85)]
 
 
-@needs_liftref
 def test_live_estimate_dist2():
     for xyz in _dist2_cases():
         for period, rng_, pct in DIST2_PARAMS:
@@ -372,12 +351,11 @@ def _qw_structures():
     return out
 
 
-@needs_ref
 def test_live_quant_weight_variants():
     for preds, npl in _qw_structures():
         for nw in ((256, 128, 64), (1, 1, 1), (8192, 0, 5)):
-            assert np.array_equal(ref_quant_weights_fixed(preds, nw), oracle_quant_weights_fixed(preds, nw))
+            assert same(ref_quant_weights_fixed(preds, nw), oracle_quant_weights_fixed(preds, nw))
         n = len(preds)
         for num_points, min_log2 in ((n, 0), (n, 2), (3 * n + 7, 1)):
-            assert np.array_equal(ref_quant_weights_scalable(preds, npl, num_points, min_log2),
-                                  oracle_quant_weights_scalable(npl, num_points, min_log2))
+            assert same(ref_quant_weights_scalable(preds, npl, num_points, min_log2),
+                        oracle_quant_weights_scalable(npl, num_points, min_log2))

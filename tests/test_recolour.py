@@ -1,7 +1,7 @@
 """Recolouring (attribute transfer to the coded geometry, SURVEY 8f N3b):
-the C oracle against the compiled reference (tolerance: the two differ only in
-how distance ties are broken), the product's kernel bodies run on the host
-against the oracle (bit-exact), and -- on a GPU -- the CUDA path against the
+the C oracle against the recorded outputs of the compiled reference
+(tolerance: the two differ only in how distance ties are broken), the
+product's kernel bodies run on the host against the oracle (bit-exact), and -- on a GPU -- the CUDA path against the
 oracle (bit-exact)."""
 import numpy as np
 import pytest
@@ -59,8 +59,6 @@ def test_oracle_vs_reference(name):
     equally near neighbour carries a different texture sample (+-20 here), so
     the comparison is a tolerance.  Measured: 71 - 100 % of the target points
     identical, mean absolute difference 0 - 1.5 levels, largest 45 levels."""
-    if not recolourref_available():
-        pytest.skip("compiled reference not present")
     sx, sa, scale, off, tx, p = _case(name)
     r = ref_recolour(p, sx, sa, scale, off, tx)
     o = oracle_recolour(p, sx, sa, scale, off, tx)
@@ -76,8 +74,6 @@ def test_oracle_vs_reference_smooth_field():
     equidistant neighbours is taken, the transferred value moves with the local
     gradient of the field only (measured: mean 0.34 levels, largest 16 on this
     sparse 8-bit shell)"""
-    if not recolourref_available():
-        pytest.skip("compiled reference not present")
     xyz, rgb = cloud_shell(6000, bits=8, seed=11)
     tx = coded_geometry(xyz, 0.5)
     p = make_recolour_params()
@@ -91,8 +87,6 @@ def test_reference_exact_without_ties():
     """on a cloud in general position (distinct irrational-ish distances: a
     non-unit scale and jittered coordinates) no tie reaches the k-th neighbour
     and the oracle reproduces the reference exactly"""
-    if not recolourref_available():
-        pytest.skip("compiled reference not present")
     rng = np.random.default_rng(5)
     sx = rng.integers(0, 4000, size=(5000, 3)).astype(np.int32)
     sx = np.unique(sx, axis=0)

@@ -67,22 +67,21 @@ def main():
         rr, rc = ref_raht(1, params, qs, mort, a_s, qpoffs=q)
         orc, oc = oracle_raht(1, params, qs, mort, a_s, qpoffs=q)
         er, ec = emu_raht(1, params, qs, mort, a_s, qpoffs=q)
-        ok = (np.array_equal(rr, orc) and np.array_equal(rc, oc) and np.array_equal(er, orc)
-              and np.array_equal(ec, oc))
+        ok = same(rr, orc) and same(rc, oc) and np.array_equal(er, orc) and np.array_equal(ec, oc)
         if ok:  # decoders from the encoder's coefficients
             dr, _ = ref_raht(0, params, qs, mort, a_s * 0, coeffs=rc, qpoffs=q)
-            do, _ = oracle_raht(0, params, qs, mort, a_s * 0, coeffs=rc, qpoffs=q)
-            de, _ = emu_raht(0, params, qs, mort, a_s * 0, coeffs=rc, qpoffs=q)
-            ok = np.array_equal(dr, do) and np.array_equal(de, do) and np.array_equal(dr, rr)
-        if ok and qpo is None and qkw["bitdepth"] <= 10 and liftref_available():
+            do, _ = oracle_raht(0, params, qs, mort, a_s * 0, coeffs=oc, qpoffs=q)
+            de, _ = emu_raht(0, params, qs, mort, a_s * 0, coeffs=oc, qpoffs=q)
+            ok = same(dr, do) and np.array_equal(de, do) and same(dr, rr)
+        if ok and qpo is None and qkw["bitdepth"] <= 10:
             # attribute level: the reference encoder's bitstream from the oracle's symbols
             payload, recon = ref_raht_encode_payload(params, qs, xyz, attrs, bitdepth=qkw["bitdepth"])
             runs, vals, ctx, tail = oracle_coeff_symbols(oc)
             out = np.empty_like(orc)
             out[order] = np.clip(orc, 0, (1 << qkw["bitdepth"]) - 1)
-            ok = (np.array_equal(out, recon)
-                  and ref_symbols_payload(0, runs, vals, ctx, tail, len(xyz)) == payload
-                  and ref_symbols_payload(1, runs, vals, ctx, tail, len(xyz)) == payload)
+            ok = (same(out, recon)
+                  and same(ref_symbols_payload(0, runs, vals, ctx, tail, len(xyz)), payload)
+                  and same(ref_symbols_payload(1, runs, vals, ctx, tail, len(xyz)), payload))
             es = emu_coeff_symbols(ec)
             ok = ok and np.array_equal(es[0], runs) and np.array_equal(es[1], vals) and es[3] == tail
         if not ok:

@@ -41,7 +41,7 @@ def main():
         rp, ri, rn = ref_lod_build(lp, xyz)
         op, oi, on = oracle_lod_build(lp, xyz)
         ep, ei, en = emu_lod_build(lp, xyz)
-        ok = (np.array_equal(rn, on) and np.array_equal(ri, oi) and np.array_equal(rp, op)
+        ok = (same(rn, on) and same(ri, oi) and same(rp, op)
               and np.array_equal(en, on) and np.array_equal(ei, oi) and np.array_equal(ep, op))
         if ok and lifting and len(xyz) > 1:
             a = int(rng.choice([1, 3]))
@@ -52,10 +52,9 @@ def main():
             ov, orr, ol = oracle_lift_encode(lp, qs, lcp, xyz, at)
             ev, er, el = emu_attr_lift(1, lp, qs, lcp, xyz, at)
             ok = np.array_equal(ev, ov) and np.array_equal(er, orr) and (not (a == 3 and lcp) or np.array_equal(el, ol))
-            if ok and liftref_available():  # the reference's own lifting encoder bodies
+            if ok:  # the reference's own lifting encoder bodies
                 rv, rrec, rl = ref_lift_encode(lp, qs, lcp, xyz, at)
-                ok = np.array_equal(rv, ov) and np.array_equal(rrec, orr) and (
-                    not (a == 3 and lcp) or np.array_equal(rl, ol))
+                ok = same(rv, ov) and same(rrec, orr) and (not (a == 3 and lcp) or same(rl, ol))
         if not ok:
             bad += 1
             print("MISMATCH case", i, "n", len(xyz), kw, "lifting", lifting)

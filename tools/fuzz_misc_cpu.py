@@ -29,13 +29,13 @@ def main():
         r, rb = ref_xyz_to_rpl(origin, theta, xyz)
         o, ob = oracle_xyz_to_rpl(origin, theta, xyz)
         e, eb = emu_xyz_to_rpl(origin, theta, xyz)
-        ok = np.array_equal(r, o) and np.array_equal(rb, ob) and np.array_equal(e, o) and np.array_equal(eb, ob)
+        ok = same(r, o) and same(rb, ob) and np.array_equal(e, o) and np.array_equal(eb, ob)
         w = ref_normalised_axes_weights(np.maximum(rb[3:], 1), 0)
         mp = rb[:3] if rng.integers(0, 2) else tuple(int(x) for x in rng.integers(-500, 500, 3))
         rs = ref_offset_and_scale(mp, w, r)
-        ok = ok and np.array_equal(rs, oracle_offset_and_scale(mp, w, o))
+        ok = ok and same(rs, oracle_offset_and_scale(mp, w, o))
         es, _ = emu_xyz_to_rpl(origin, theta, xyz, weight=w, min_pos=mp)
-        ok = ok and np.array_equal(es, rs)
+        ok = ok and same(es, rs)
         # estimateDist2 on the Morton-sorted cloud (non-negative coordinates)
         pos = np.abs(xyz)
         _, _, order = sort_cloud(pos, np.zeros((n, 1), dtype=np.int32))
@@ -49,12 +49,11 @@ def main():
         preds, npl = synth_predictors(m, int(rng.integers(2, 9)), seed=int(rng.integers(1 << 30)))
         nw = tuple(int(x) for x in rng.integers(0, 600, 3))
         qr = ref_quant_weights_fixed(preds, nw)
-        ok = ok and np.array_equal(qr, oracle_quant_weights_fixed(preds, nw)) and np.array_equal(
-            qr, emu_quant_weights_fixed(preds, npl, nw))
+        ok = ok and same(qr, oracle_quant_weights_fixed(preds, nw), emu_quant_weights_fixed(preds, npl, nw))
         numpts, ml2 = int(rng.integers(m, 4 * m)), int(rng.integers(0, 3))
         sr_ = ref_quant_weights_scalable(preds, npl, numpts, ml2)
-        ok = ok and np.array_equal(sr_, oracle_quant_weights_scalable(npl, numpts, ml2)) and np.array_equal(
-            sr_, emu_quant_weights_scalable(npl, numpts, ml2))
+        ok = ok and same(sr_, oracle_quant_weights_scalable(npl, numpts, ml2),
+                         emu_quant_weights_scalable(npl, numpts, ml2))
         if not ok:
             bad += 1
             print("MISMATCH case", i, "n", n, "bits", bits, "lasers", nt, "origin", origin, period, sr, pct, nw)
